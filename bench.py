@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--series S] [--len L]
                     [--settings comprehensive|efficient|minimal] [--placement auto|copy|store|multicast|nccl]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (ComprehensiveFCParameters, 783 columns) over one batch of S synthetic
 series of length L per GPU (default 1 000 000 x 256 = BASELINE.json configs[2], the configuration the
@@ -20,6 +21,13 @@ same run: config2 (Efficient 100 k x 256, N = 1), config4 (Comprehensive 1 M x 1
 config5 (roll_time_series 10 k x 4096 -> 1.21 M window views, sharded by parent), minimal (the reduction-only
 kernel behind `roofline.minimal`).
 `--impl reference` times the CPU path (the oracle port of the reference, all host cores) instead.
+`--dump-outputs DIR` writes what the last timed step of the headline pass left in the feature matrix, so that two builds
+can be compared output for output (the inputs are seeded).  DUMP_ROWS rows of the [N*S, F] matrix are drawn with a fixed
+seed (all rows when there are fewer); every file holds finite values only:
+  DIR/features.npy            float64 [rows, F]  the features, 0 where the feature is not finite
+  DIR/features_nonfinite.npy  float32 [rows, F]  0 finite, 1 NaN, 2 +inf, 3 -inf (some features are NaN by definition,
+                                                 e.g. query_similarity_count without a query)
+  DIR/features_rows.npy       float64 [rows]     the row numbers, ascending
 """
 import argparse
 import json
@@ -35,6 +43,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "series/sec extract_features ComprehensiveFCParameters"
+DUMP_ROWS = 6144        # x 783 columns x (8 + 4) bytes = 58 MB: the largest plan's dump stays under 64 MB
 
 
 def settings_by_name(name):
@@ -307,9 +316,10 @@ class Bench:
         return self.torch.randn(shape, generator=gen, device=self.dev, dtype=self.torch.float32)
 
 
-def sharded_pass(B, name, values, S, L, steps, warmup, csr=None, placement="auto", rows_alloc=None):
+def sharded_pass(B, name, values, S, L, steps, warmup, csr=None, placement="auto", rows_alloc=None, on_timed=None):
     """One configuration, device-resident: every rank extracts its S series (dense [S, L] tensor, or a CSR
     (begin, length) over `values`) and the rows are placed on every rank (tsfresh_b200.distributed.GatheredMatrix).
+    on_timed(gm) is called once the timed steps have finished, before anything else writes the matrix.
     Returns (ms per step max over ranks, per-group ms of one extra timed pass over this rank's shard, launches/step, gm)."""
     from tsfresh_b200.distributed import GatheredMatrix, extract_csr_sharded_device, extract_dense_sharded_device
     torch = B.torch
@@ -328,6 +338,8 @@ def sharded_pass(B, name, values, S, L, steps, warmup, csr=None, placement="auto
             gm.finish(B.ctx, stream=B.stream, ctx_on_current_stream=True)
 
     ms = B.timed(step, steps, warmup)
+    if on_timed is not None:
+        on_timed(gm)
     launches = B.ctx.launch_count() * blocks[0]
     gm.detach(B.ctx)
     # per-group CUDA events: one extra pass over this rank's whole shard with TSFX_FLAG_TIMING
@@ -355,7 +367,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="headline configuration only")
     ap.add_argument("--placement", default="auto", choices=["auto", "copy", "store", "multicast", "nccl"])
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's feature matrix here")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's feature matrix; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -372,8 +389,9 @@ def main():
     sampler = ClockSampler(B.local_rank)
     if rank == 0:
         sampler.start()
+    dump = (lambda gm: dump_outputs(args.dump_outputs, gm)) if args.dump_outputs and rank == 0 else None
     ms_step, group_ms, launches_per_step, gm = sharded_pass(B, args.settings, values, S, L, args.steps, args.warmup,
-                                                           placement=args.placement)
+                                                           placement=args.placement, on_timed=dump)
     clocks = sampler.stop() if rank == 0 else None
     value = world * S / (ms_step / 1e3)
     placement = gm.placement()
@@ -620,6 +638,22 @@ def main():
         if B.saved_stdout is not None and rank != 0:
             os.dup2(B.saved_stdout, 1)
         dist.destroy_process_group()
+
+
+def dump_outputs(directory, gm):
+    """DUMP_ROWS rows of gm.full (all rows when there are fewer), drawn with a fixed seed -> directory/*.npy"""
+    import torch
+    n = gm.full.shape[0]
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    sample = gm.full.index_select(0, torch.from_numpy(rows).to(gm.full.device)).cpu().numpy()
+    code = np.zeros(sample.shape, np.float32)
+    code[np.isnan(sample)] = 1
+    code[sample == np.inf] = 2
+    code[sample == -np.inf] = 3
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "features.npy"), np.where(code == 0, sample, 0.0))
+    np.save(os.path.join(directory, "features_nonfinite.npy"), code)
+    np.save(os.path.join(directory, "features_rows.npy"), rows.astype(np.float64))
 
 
 def group_columns(plan):

@@ -1,208 +1,180 @@
-"""Pins the oracle (oracle/calculators.py) and the plan compiler's column names against the UNMODIFIED
-reference imported from /root/reference (build container only; skipped on the GPU box)."""
+"""Pins the oracle (oracle/calculators.py) and the plan compiler's column names against the UNMODIFIED reference.
+
+The reference's answers are stored in tests/golden/reference.npz and tests/golden/reference.json (written by
+`python -m oracle.make_golden_reference`, which needs the reference tree); the inputs are regenerated here from the
+same seeds."""
+import ast
+import builtins
+import json
+import os
 import warnings
 
 import numpy as np
 import pandas as pd
 import pytest
 
-from oracle import ref_shim
 from oracle.extract import compare, oracle_rows
+from oracle.make_golden_reference import (FRAME_CASES, IMPUTE_CASES, ROLL_CASES, ROLLING_TESTS, TIMEWISE_LENGTHS,
+                                          from_columns_input, impute_input, normalise_kind_to_fc, roll_frame,
+                                          short_series, timewise_series)
 from tests.helpers import synthetic_series
 from tsfresh_b200.plan import Plan
 from tsfresh_b200.settings import ComprehensiveFCParameters, EfficientFCParameters, MinimalFCParameters
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-def reference_frame(series, settings):
-    ref_shim.load()
-    from tsfresh.feature_extraction import extract_features
-    ids = np.concatenate([np.full(len(s), i) for i, s in enumerate(series)])
-    t = np.concatenate([np.arange(len(s)) for s in series])
-    v = np.concatenate([np.asarray(s, np.float32).astype(np.float64) for s in series])
-    df = pd.DataFrame({"id": ids, "time": t, "value": v})
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        return extract_features(df, column_id="id", column_sort="time", default_fc_parameters=settings, n_jobs=0,
-                                disable_progressbar=True)
+@pytest.fixture(scope="module")
+def npz():
+    with np.load(os.path.join(GOLDEN, "reference.npz"), allow_pickle=False) as z:
+        return dict(z)
 
 
-def test_settings_match_reference():
-    ref_shim.load()
-    from tsfresh.feature_extraction import settings as rs
-    for mine, theirs in ((ComprehensiveFCParameters(), rs.ComprehensiveFCParameters()),
-                         (EfficientFCParameters(), rs.EfficientFCParameters()),
-                         (MinimalFCParameters(), rs.MinimalFCParameters())):
+@pytest.fixture(scope="module")
+def js():
+    with open(os.path.join(GOLDEN, "reference.json")) as f:
+        return json.load(f)
+
+
+def test_settings_match_reference(js):
+    for mine, name in ((ComprehensiveFCParameters(), "comprehensive"), (EfficientFCParameters(), "efficient"),
+                       (MinimalFCParameters(), "minimal")):
+        theirs = {k: ast.literal_eval(v) for k, v in js["settings"][name]}
         assert list(mine.keys()) == list(theirs.keys())
         for k in mine:
             assert mine[k] == theirs[k], k
 
 
-@pytest.mark.parametrize("kind,length,count", [("normal", 256, 6), ("walk", 100, 4), ("rounded", 64, 4), ("normal", 1300, 2)])
-def test_oracle_matches_reference(kind, length, count):
+@pytest.mark.parametrize("kind,length,count", FRAME_CASES)
+def test_oracle_matches_reference(npz, kind, length, count):
     series = list(synthetic_series(11, count, length, kind))
     settings = ComprehensiveFCParameters()
-    X = reference_frame(series, settings)
+    key = "frame_%s_%d_%d" % (kind, length, count)
     plan = Plan(settings)
-    assert ["value__" + s for s in plan.suffixes] == list(X.columns)
+    assert ["value__" + s for s in plan.suffixes] == list(npz[key + "_columns"])
     mine = oracle_rows([s.astype(np.float64) for s in series], settings)
-    bad = compare(mine, X.to_numpy(dtype=np.float64), plan.suffixes, rtol=1e-12)
+    bad = compare(mine, npz[key], plan.suffixes, rtol=1e-12)
     assert not bad, bad[:20]
 
 
-def test_oracle_matches_reference_short_series():
-    rng = np.random.default_rng(3)
-    series = [rng.standard_normal(n).astype(np.float32) for n in (1, 2, 3, 4, 5, 8, 12, 20, 23, 31, 40)]
-    series += [np.zeros(9, np.float32), np.ones(5, np.float32), np.array([1, 1, 2, 2, 3, 3, 3], np.float32)]
+def test_oracle_matches_reference_short_series(npz):
+    series = short_series()
     settings = ComprehensiveFCParameters()
-    X = reference_frame(series, settings)
     plan = Plan(settings)
     mine = oracle_rows([s.astype(np.float64) for s in series], settings)
-    bad = compare(mine, X.to_numpy(dtype=np.float64), plan.suffixes, rtol=1e-12)
+    bad = compare(mine, npz["frame_short"], plan.suffixes, rtol=1e-12)
     assert not bad, bad[:20]
 
 
-def test_oracle_impute_matches_reference():
+def test_oracle_impute_matches_reference(npz):
     """oracle/impute.py against tsfresh.utilities.dataframe_functions (:49-212) on random matrices."""
-    ref_shim.load()
-    from tsfresh.utilities import dataframe_functions as rdf
     from oracle import impute as oi
-    from oracle.make_golden_impute import make_input
-    for seed, rows, cols in ((1, 50, 9), (2, 201, 14), (3, 17, 11)):
-        m = make_input(seed, rows, cols) if cols >= 10 else np.random.default_rng(seed).standard_normal((rows, cols))
-        names = ["c%d" % i for i in range(m.shape[1])]
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            cmax, cmin, cmed = rdf.get_range_values_per_column(pd.DataFrame(m.copy(), columns=names))
-            want = rdf.impute(pd.DataFrame(m.copy(), columns=names)).to_numpy(np.float64)
-            want0 = rdf.impute_dataframe_zero(pd.DataFrame(m.copy(), columns=names)).to_numpy(np.float64)
+    for seed, rows, cols in IMPUTE_CASES:
+        m = impute_input(seed, rows, cols)
         st = oi.range_values(m)
-        assert np.array_equal(st[0], [cmin[c] for c in names])
-        assert np.array_equal(st[1], [cmax[c] for c in names])
-        assert np.array_equal(st[2], [float(cmed[c]) for c in names])
-        assert np.array_equal(oi.impute(m), want)
-        assert np.array_equal(oi.impute_zero(m), want0)
+        want = npz["impute%d_range" % seed]
+        assert np.array_equal(st[0], want[0])
+        assert np.array_equal(st[1], want[1])
+        assert np.array_equal(st[2], want[2])
+        assert np.array_equal(oi.impute(m), npz["impute%d" % seed])
+        assert np.array_equal(oi.impute_zero(m), npz["impute%d_zero" % seed])
 
 
-def test_roll_time_series_views_reproduce_reference_frame():
+def test_roll_time_series_views_reproduce_reference_frame(npz):
     """tsfresh_b200.roll_time_series(...).to_frame() == the reference's materialised rolled frame (ids, row order,
     values) for both directions, shuffled input and a missing sort column."""
-    ref_shim.load()
-    from tsfresh.utilities.dataframe_functions import roll_time_series as ref_roll
     from tsfresh_b200 import roll_time_series
-    rng = np.random.default_rng(3)
-    lens = [20, 9, 31, 1, 2]
-    df = pd.DataFrame({"id": np.concatenate([np.full(n, i * 10) for i, n in enumerate(lens)]),
-                       "time": np.concatenate([np.arange(n) * 2 + 5 for n in lens]),
-                       "a": rng.standard_normal(sum(lens)).astype(np.float32),
-                       "b": rng.standard_normal(sum(lens)).astype(np.float32)})
+    df = roll_frame()
     for shuffle in (False, True):
         d = df.sample(frac=1.0, random_state=1).reset_index(drop=True) if shuffle else df
-        for rd, mx, mn in [(-1, 7, 0), (-3, 7, 7), (3, 7, 0), (1, None, 3), (2, 4, 4)]:
-            with warnings.catch_warnings():
-                warnings.simplefilter("ignore")
-                want = ref_roll(d.copy(), column_id="id", column_sort="time", rolling_direction=rd, max_timeshift=mx,
-                                min_timeshift=mn, n_jobs=0, disable_progressbar=True).reset_index(drop=True)
+        for k, (rd, mx, mn) in enumerate(ROLL_CASES):
+            key = "roll%d_%d" % (int(shuffle), k)
             got = roll_time_series(d, column_id="id", column_sort="time", rolling_direction=rd, max_timeshift=mx,
                                    min_timeshift=mn).to_frame()
-            assert list(want["id"]) == list(got["id"]), (shuffle, rd, mx, mn)
-            assert np.array_equal(want["time"], got["time"])
+            assert [tuple(i) for i in npz[key + "_id"].tolist()] == list(got["id"]), (shuffle, rd, mx, mn)
+            assert np.array_equal(npz[key + "_time"], got["time"])
             for c in "ab":
-                assert np.array_equal(want[c].to_numpy(np.float32), got[c])
+                assert np.array_equal(npz[key + "_" + c], got[c])
     d = df.drop(columns=["time"])
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        want = ref_roll(d.copy(), column_id="id", rolling_direction=2, max_timeshift=5, n_jobs=0, disable_progressbar=True)
     got = roll_time_series(d, column_id="id", rolling_direction=2, max_timeshift=5).to_frame()
-    assert list(want["id"]) == list(got["id"]) and np.array_equal(want["sort"].to_numpy(), got["sort"].to_numpy())
+    assert [tuple(i) for i in npz["roll_nosort_id"].tolist()] == list(got["id"])
+    assert np.array_equal(npz["roll_nosort_sort"], got["sort"].to_numpy())
 
 
-def test_reference_rolling_test_cases_pass_on_the_view_implementation():
-    """The reference's own RollingTestCase (tests/units/utilities/test_dataframe_functions.py:18-944) run against
-    tsfresh_b200.roll_time_series(...).to_frame(): positive / negative / larger-shift / stacked (kind column) / dict /
-    order / warning / validation cases."""
-    import importlib.util
-    import os
-    import unittest
-    ref_shim.load()
-    from tsfresh.utilities import dataframe_functions as rdf
-    from tsfresh_b200 import roll_time_series as mine
+def _frame(cols):
+    return pd.DataFrame({c["name"]: pd.Series(c["values"], dtype=c["dtype"]) for c in cols})
 
-    def adapter(df_or_dict, column_id, column_sort=None, column_kind=None, rolling_direction=1, max_timeshift=None,
-                min_timeshift=0, **kw):
-        r = mine(df_or_dict, column_id, column_sort=column_sort, column_kind=column_kind,
-                 rolling_direction=rolling_direction, max_timeshift=max_timeshift, min_timeshift=min_timeshift,
-                 show_warnings=True)
-        return {k: v.to_frame() for k, v in r.items()} if isinstance(r, dict) else r.to_frame()
 
-    import sys
-    original = rdf.roll_time_series
-    rdf.roll_time_series = adapter
-    # the reference test module does `from tests.fixtures import warning_free`; `tests` is THIS repo's package here
-    fspec = importlib.util.spec_from_file_location("ref_tests_fixtures", os.path.join(ref_shim.REFERENCE_ROOT, "tests", "fixtures.py"))
-    fixtures = importlib.util.module_from_spec(fspec)
-    fspec.loader.exec_module(fixtures)
-    saved_fixtures = sys.modules.get("tests.fixtures")
-    sys.modules["tests.fixtures"] = fixtures
-    try:
-        path = os.path.join(ref_shim.REFERENCE_ROOT, "tests", "units", "utilities", "test_dataframe_functions.py")
-        spec = importlib.util.spec_from_file_location("ref_test_dataframe_functions", path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        names = ["test_with_wrong_input", "test_assert_single_row", "test_positive_rolling", "test_negative_rolling",
-                 "test_rolling_with_larger_shift", "test_stacked_rolling", "test_dict_rolling",
-                 "test_dict_rolling_maxshift_1", "test_order_rolling", "test_warning_on_non_uniform_time_steps"]
-        suite = unittest.TestSuite(mod.RollingTestCase(n) for n in names)
-        res = unittest.TextTestRunner(verbosity=0).run(suite)
-        assert res.testsRun == len(names) and res.wasSuccessful(), (res.failures, res.errors)
-    finally:
-        rdf.roll_time_series = original
-        if saved_fixtures is None:
-            sys.modules.pop("tests.fixtures", None)
+def _assert_frame_matches(got, want_cols, column_id, where):
+    for c in want_cols:
+        if c["name"] == column_id != "id":
+            continue            # the reference keeps the parent id column; here it is the first element of the "id" pairs
+        assert c["name"] in got.columns, (where, c["name"])
+        g = list(got[c["name"]])
+        if c["tuples"]:
+            assert g == [tuple(v) for v in c["values"]], (where, c["name"])
+        elif pd.api.types.is_numeric_dtype(c["dtype"]):
+            assert np.array_equal(np.asarray(g, np.float64), np.asarray(c["values"], np.float64), equal_nan=True), \
+                (where, c["name"])
         else:
-            sys.modules["tests.fixtures"] = saved_fixtures
+            assert g == c["values"], (where, c["name"])
 
 
-def test_from_columns_matches_reference():
+def test_reference_rolling_test_cases_pass_on_the_view_implementation(js):
+    """Every roll_time_series call of the reference's own RollingTestCase (tests/units/utilities/
+    test_dataframe_functions.py:18-944) replayed on tsfresh_b200.roll_time_series(...).to_frame(): positive / negative /
+    larger-shift / stacked (kind column) / dict / order / warning / validation cases give the frames, exception types
+    and warnings the reference gave."""
+    from tsfresh_b200 import roll_time_series as mine
+    cases = js["rolling_test_case"]
+    assert [c["test"] for c in cases] == ROLLING_TESTS
+    for case in cases:
+        assert case["calls"], case["test"]
+        for n, call in enumerate(case["calls"]):
+            where = (case["test"], n)
+            data = ({k: _frame(v) for k, v in call["input"].items()} if call["input_is_dict"] else _frame(call["input"]))
+            if "raises" in call:
+                with pytest.raises(getattr(builtins, call["raises"])):
+                    mine(data, show_warnings=True, **call["kwargs"])
+                continue
+            with warnings.catch_warnings(record=True) as caught:
+                warnings.simplefilter("always")
+                r = mine(data, show_warnings=True, **call["kwargs"])
+            messages = {str(w.message) for w in caught}
+            for m in call["warnings"]:
+                assert m in messages, (where, m)
+            if call["input_is_dict"]:
+                assert isinstance(r, dict) and sorted(r) == sorted(call["output"]), where
+                for k, want in call["output"].items():
+                    _assert_frame_matches(r[k].to_frame(), want, call["kwargs"]["column_id"], where + (k,))
+            else:
+                _assert_frame_matches(r.to_frame(), call["output"], call["kwargs"]["column_id"], where)
+
+
+def test_from_columns_matches_reference(js):
     """settings.from_columns (settings.py:23-83): same kind_to_fc_parameters and same errors as the reference."""
-    ref_shim.load()
-    from tsfresh.feature_extraction import settings as rs
     from tsfresh_b200.settings import from_columns
-    cols = (["value__" + s for s in Plan(ComprehensiveFCParameters()).suffixes]
-            + ["other__maximum", "other__quantile__q_0.25", 'k__agg_linear_trend__attr_"slope"__chunk_len_5__f_agg_"max"',
-               "k__value_count__value_nan", "k__range_count__max_inf__min_-inf", "k__fft_coefficient__attr_\"abs\"__coeff_3"])
-    mine = from_columns(cols + ["skipme"], columns_to_ignore=["skipme"])
-    ref = rs.from_columns(cols + ["skipme"], columns_to_ignore=["skipme"])
-
-    def norm(d):
-        return {k: {f: (None if p is None else [tuple(sorted((a, repr(b)) for a, b in q.items())) for q in p])
-                    for f, p in v.items()} for k, v in d.items()}
-    assert norm(mine) == norm(ref) and list(mine) == list(ref)
-    for bad, err in ((["nounderscore"], ValueError), ([3], TypeError), (["value__not_a_calculator"], ValueError)):
+    ref = js["from_columns"]
+    mine = from_columns(from_columns_input() + ["skipme"], columns_to_ignore=["skipme"])
+    assert normalise_kind_to_fc(mine) == ast.literal_eval(ref["parsed"]) and list(mine) == ref["kinds"]
+    expected = [(["nounderscore"], ValueError), ([3], TypeError), (["value__not_a_calculator"], ValueError)]
+    assert [[bad, err.__name__] for bad, err in expected] == ref["errors"]
+    for bad, err in expected:
         with pytest.raises(err):
             from_columns(bad)
-        with pytest.raises(err):
-            rs.from_columns(bad)
 
 
-def test_linear_trend_timewise_matches_reference():
+def test_linear_trend_timewise_matches_reference(npz):
     """feature_calculators.py:2274-2306 with its own known answers (test_feature_calculations.py:1796-1935) and on
     irregularly sampled random series"""
-    import pandas as pd
     from oracle import calculators as C
-    ref = ref_shim.load()
-    from tsfresh.feature_extraction.feature_calculators import linear_trend_timewise
     param = [{"attr": a} for a in ("pvalue", "rvalue", "intercept", "slope", "stderr")]
     x = pd.Series([0, 1, 3, 6], index=pd.DatetimeIndex(["2018-01-01 04:00:00", "2018-01-01 05:00:00", "2018-01-01 07:00:00",
                                                          "2018-01-01 10:00:00"]))
     got = C.linear_trend_timewise(x.to_numpy(), x.index.as_unit("ns").asi8, param)
     assert got[3] == pytest.approx(1.0, abs=1e-3) and got[2] == pytest.approx(0.0, abs=1e-3)
     rng = np.random.default_rng(12)
-    for n in (2, 3, 17, 256):
-        gaps = rng.integers(1, 5000, n).cumsum() * 10 ** 9 + rng.integers(0, 10 ** 9, n)
-        ix = pd.DatetimeIndex(np.sort(gaps).astype("datetime64[ns]"))
-        s = pd.Series(rng.standard_normal(n).astype(np.float32).astype(np.float64), index=ix)
-        want = [v for _, v in linear_trend_timewise(s, param)]
-        got = C.linear_trend_timewise(s.to_numpy(), ix.asi8, param)
-        np.testing.assert_allclose(got, want, rtol=1e-12, equal_nan=True)
+    for n in TIMEWISE_LENGTHS:
+        s = timewise_series(rng, n)
+        got = C.linear_trend_timewise(s.to_numpy(), s.index.asi8, param)
+        np.testing.assert_allclose(got, npz["timewise%d" % n], rtol=1e-12, equal_nan=True)
