@@ -898,11 +898,10 @@ cudaError_t launch_basic(const BasicArgs& A0, int max_len, cudaStream_t st, int 
     A.npad = (max_len + 3) & ~3;
     A.nxc = ((max_len + 255) / 256) * 256 + ((A.lag_needed + 1) & ~1);      // centred copy + zero tail for the lag products
     {
-        // lag products on the FP64 tensor cores (DMMA) unless TSFX_LAG=fma or the largest lag needs more than 8 tiles
-        static int mode = -1;
-        if (mode < 0) { const char* e = getenv("TSFX_LAG"); mode = (e && e[0] == 'f') ? 0 : 1; }
+        // lag products on the FP64 tensor cores (DMMA) unless the largest lag needs more than TSFX_DMMA_MAX_TILES tiles
+        // (then the FMA path); measured on B200 at 1 M x 256: 53.2 ms (FMA) -> 52.5 ms (DMMA) for the whole kernel
         const int tiles = A.lag_needed / 8 + 1 + ((A.lag_needed & 7) ? 1 : 0);
-        A.lag_tiles = (mode == 1 && A.lag_needed > 0 && tiles <= TSFX_DMMA_MAX_TILES) ? tiles : 0;
+        A.lag_tiles = (A.lag_needed > 0 && tiles <= TSFX_DMMA_MAX_TILES) ? tiles : 0;
         if (A.lag_tiles > 0) {     // the strided fragment loads read up to 32 ceil(n / 32) + 8 tiles + 24 samples
             const int need = ((max_len + 31) / 32) * 32 + 8 * A.lag_tiles + 32;
             if (A.nxc < need) A.nxc = (need + 1) & ~1;
@@ -918,31 +917,17 @@ cudaError_t launch_basic(const BasicArgs& A0, int max_len, cudaStream_t st, int 
     A.gscratch = G.gscratch;
     G.smem += A.desc_bytes;                       // CTA-wide descriptor table in front of the per-warp regions
     if (G.smem > 227 * 1024) return cudaErrorInvalidConfiguration;
-    {
-        // Two CTAs of 12 warps per SM instead of three of 8 (TSFX_BASIC_WPC=8|12|24): all warps of a CTA walk the descriptor
-        // list in lock step, so larger CTAs share more of the 250 KB instruction stream -- measured on B200 at 1 M x 256:
-        // 52.5 ms (3 x 8) -> 42.9 ms (2 x 12), 43.9 ms (1 x 24); stall_no_instruction was the top stall reason
-        static int wide = -1;
-        if (wide < 0) { const char* e = getenv("TSFX_BASIC_WPC"); wide = e ? atoi(e) : 12; }
-        if ((wide == 12 || wide == 24) && !G.gscratch && G.wpc == 8) {
-            const size_t smem = per * wide + A.desc_bytes;
-            if (smem <= 227 * 1024) {
-                const int64_t ctas = (A.R.n_series + wide - 1) / wide;
-                const int64_t cap = (int64_t)sm_count * grid_waves(4096);
-                const int grid = (int)std::max<int64_t>(1, std::min(ctas, cap));
-                cudaError_t e;
-                if (wide == 12) {
-                    e = cudaFuncSetAttribute(k_basic<12, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                    if (e != cudaSuccess) return e;
-                    k_basic<12, false><<<grid, 12 * 32, smem, st>>>(A);
-                } else {
-                    e = cudaFuncSetAttribute(k_basic<24, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                    if (e != cudaSuccess) return e;
-                    k_basic<24, false><<<grid, 24 * 32, smem, st>>>(A);
-                }
-                return cudaGetLastError();
-            }
-        }
+    if (!G.gscratch && G.wpc == 8 && per * 12 + A.desc_bytes <= 227 * 1024) {
+        // Two CTAs of 12 warps per SM instead of three of 8: all warps of a CTA walk the descriptor list in lock step,
+        // so larger CTAs share more of the 250 KB instruction stream -- measured on B200 at 1 M x 256: 52.5 ms (3 x 8)
+        // -> 42.9 ms (2 x 12), 43.9 ms (1 x 24); stall_no_instruction was the top stall reason
+        const size_t smem = per * 12 + A.desc_bytes;
+        const int64_t ctas = (A.R.n_series + 11) / 12;
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ctas, (int64_t)sm_count * 4096));
+        cudaError_t e = cudaFuncSetAttribute(k_basic<12, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        k_basic<12, false><<<grid, 12 * 32, smem, st>>>(A);
+        return cudaGetLastError();
     }
     TSFX_DISPATCH(k_basic, G, st, A)
     return cudaGetLastError();

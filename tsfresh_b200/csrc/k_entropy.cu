@@ -5,85 +5,33 @@
 // Chebyshev distance is <= tau, for templates of length 2 (i, j in [0, n-2]) and of length 3
 // (i, j in [0, n-3]).  One warp per series; up to NT = 6 tolerances share one pass so the distances are formed
 // once.  Differences are float64 of float32-origin values, i.e. the very same IEEE operations numpy performs,
-// so the counts are bit-identical to the reference's.  Three formulations of the counting (TSFX_ENTROPY selects):
-//   * rank space (default, k_entropy_rank; series of up to ~1100 samples): sort once, the matches of a sample are a
-//     contiguous rank interval, bit rows come from a prefix-bit table -- no pair tests at all (see the comment there);
-//   * bit tiles (TSFX_ENTROPY=tiles and all longer series, entropy_bittile): lane = row i, 32-column bit words per
-//     tolerance, counts by popcount of three shifted rows -- ~17 warp instructions per 32 pair tests and 6 tolerances;
-//   * pair sweep (TSFX_ENTROPY=pairs, entropy_sweep): lane = row i, sequential sweep over j with the three
-//     neighbouring samples in registers -- ~35; kept for A/B measurements and as a cross-check.
+// so the counts are bit-identical to the reference's.  Two formulations of the counting, chosen by the series length:
+//   * rank space (k_entropy_rank; series of up to ~1100 samples): sort once, the matches of a sample are a contiguous
+//     rank interval, bit rows come from a prefix-bit table -- no pair tests at all (see the comment there);
+//   * bit tiles (all longer series, entropy_bittile): lane = row i, 32-column bit words per tolerance, counts by
+//     popcount of three shifted rows -- ~17 warp instructions per 32 pair tests and 6 tolerances.
 #include <algorithm>
-#include <cstdlib>
 
 #include "tsfx_common.cuh"
 #include "tsfx_kernels.h"
 
 namespace tsfx {
 
-// c += (m <= tau) as DSETP + one predicated IADD (the compiler's own choice is VIADD + predicated MOV)
-__device__ __forceinline__ void count_le(int& c, double m, double tau) {
-    asm("{\n\t.reg .pred p;\n\tsetp.le.f64 p, %1, %2;\n\t@p add.s32 %0, %0, 1;\n\t}" : "+r"(c) : "d"(m), "d"(tau));
-}
-// max of two non-NaN magnitudes without fmax()'s NaN handling (DSETP + SEL instead of DSETP.MAX/FSEL/SEL/LOP3)
-__device__ __forceinline__ double max_nn(double a, double b) { return a > b ? a : b; }
 // |x| as one integer AND on the high word (keeps the half-rate FP64 pipe for the subtractions and compares)
 __device__ __forceinline__ double abs_bits(double x) {
     return __hiloint2double(__double2hiint(x) & 0x7fffffff, __double2loint(x));
 }
 
-template <int NT>
-__device__ __forceinline__ void entropy_sweep(const double* xd, int n, const double (&tau)[NT], double (&sum_ln2)[NT],
-                                              double (&sum_ln3)[NT], double (&sumB)[NT], double (&sumA)[NT], int lane) {
-#pragma unroll
-    for (int t = 0; t < NT; ++t) { sum_ln2[t] = 0.0; sum_ln3[t] = 0.0; sumB[t] = 0.0; sumA[t] = 0.0; }
-    const int n2 = n - 1, n3 = n - 2;          // number of length-2 / length-3 templates
-    if (n2 <= 0) return;
-    const double inv2 = 1.0 / (double)n2, inv3 = n3 > 0 ? 1.0 / (double)n3 : 0.0;
-    for (int r0 = 0; r0 < n2; r0 += 32) {
-        const int i = r0 + lane;
-        const bool v2 = i < n2, v3 = i < n3;
-        const double a0 = v2 ? xd[i] : 0.0, a1 = v2 ? xd[i + 1] : 0.0, a2 = v3 ? xd[i + 2] : 0.0;
-        int c2[NT], c3[NT];
-#pragma unroll
-        for (int t = 0; t < NT; ++t) { c2[t] = 0; c3[t] = 0; }
-        double b0 = xd[0], b1 = xd[1];
-        for (int j = 0; j < n3; ++j) {
-            const double b2 = xd[j + 2];
-            const double m2 = max_nn(abs_bits(a0 - b0), abs_bits(a1 - b1));
-            const double m3 = max_nn(m2, abs_bits(a2 - b2));
-#pragma unroll
-            for (int t = 0; t < NT; ++t) { count_le(c2[t], m2, tau[t]); count_le(c3[t], m3, tau[t]); }
-            b0 = b1; b1 = b2;
-        }
-        {   // last length-2 template j = n2 - 1
-            const double m2 = max_nn(abs_bits(a0 - b0), abs_bits(a1 - b1));
-#pragma unroll
-            for (int t = 0; t < NT; ++t) count_le(c2[t], m2, tau[t]);
-        }
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-            if (v2) { sum_ln2[t] += log((double)c2[t] * inv2); sumB[t] += (double)(c2[t] - 1); }
-            if (v3) { sum_ln3[t] += log((double)c3[t] * inv3); sumA[t] += (double)(c3[t] - 1); }
-        }
-    }
-#pragma unroll
-    for (int t = 0; t < NT; ++t) {
-        sum_ln2[t] = wsum(sum_ln2[t]);
-        sum_ln3[t] = wsum(sum_ln3[t]);
-        sumB[t] = wsum(sumB[t]);
-        sumA[t] = wsum(sumA[t]);
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------
-// Bit-tile formulation (default).  For a tolerance tau let R_i be the bit row R_i[j] = [ |x_i - x_j| <= tau ].
+// Bit-tile formulation.  For a tolerance tau let R_i be the bit row R_i[j] = [ |x_i - x_j| <= tau ].
 // The template counts are then pure bit operations on three consecutive rows:
 //     c2(i) = popc( R_i & (R_{i+1} >> 1) )                      c3(i) = popc( R_i & (R_{i+1} >> 1) & (R_{i+2} >> 2) )
 // (samples beyond n are NaN, whose comparisons are false, so the ranges j <= n-2 / j <= n-3 need no masks).
 // Lane = row i; a 32-column tile of R_i is built with one float64 subtract per pair plus one DSETP + predicated OR
 // per tolerance -- the same IEEE operations numpy performs, so the counts stay bit-identical -- and rows i+1, i+2
 // come from the neighbouring lanes by shuffle, which is why a row block advances by 30 rows, not 32.  Per 32 pairs
-// and 6 tolerances this issues ~17 warp instructions (7 of them FP64) against ~35 (17 FP64) for the pair sweep.
+// and 6 tolerances this issues ~17 warp instructions (7 of them FP64) against ~35 (17 FP64) for a sweep over j with
+// one pair test per tolerance.
 __device__ __forceinline__ void or_le(unsigned& w, double d, double tau, unsigned bit) {
     asm("{\n\t.reg .pred p;\n\tsetp.le.f64 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(w) : "d"(d), "d"(tau), "r"(bit));
 }
@@ -149,7 +97,7 @@ __device__ __forceinline__ void entropy_bittile(const double* xd, const double* 
 
 template <int NT>
 __device__ __forceinline__ void entropy_batch(const Desc* descs, int j0, int cnt, const double* xd, int n, double sd,
-                                              double* orow, int lane, const double* lnk, bool bittile) {
+                                              double* orow, int lane, const double* lnk) {
     double tau[NT], l2[NT], l3[NT], sB[NT], sA[NT];
 #pragma unroll
     for (int t = 0; t < NT; ++t) {
@@ -158,8 +106,7 @@ __device__ __forceinline__ void entropy_batch(const Desc* descs, int j0, int cnt
             tau[t] = (d.calc == TSFX_SAMPLE_ENTROPY) ? 0.2 * sd : d.p0 * sd;
         } else tau[t] = -1.0;
     }
-    if (bittile) entropy_bittile<NT>(xd, lnk, n, tau, l2, l3, sB, sA, lane);
-    else entropy_sweep<NT>(xd, n, tau, l2, l3, sB, sA, lane);
+    entropy_bittile<NT>(xd, lnk, n, tau, l2, l3, sB, sA, lane);
 #pragma unroll
     for (int t = 0; t < NT; ++t) {
         if (t < cnt) {
@@ -186,35 +133,32 @@ __global__ void __launch_bounds__(WPC * 32, (WPC == 4 ? 3 : 1)) k_entropy(Entrop
     for (int64_t s = (int64_t)blockIdx.x * WPC + warp; s < A.R.n_series; s += warps_total) {
         const int n = load_series(A.R, s, xs, lane);
         const Moments M = moments(xs, n, nullptr, lane);
-        const bool bm = A.bittile != 0;
-        // padding: NaN for the bit tiles (comparisons false), zeros at n, n+1 for the pair sweep
-        for (int i = lane; i < A.xpad; i += 32) xd[i] = i < n ? (double)xs[i] : ((bm || i >= n + 2) ? dnan() : 0.0);
-        if (bm) for (int k = lane; k <= n; k += 32) lnk[k] = log((double)k);
+        for (int i = lane; i < A.xpad; i += 32) xd[i] = i < n ? (double)xs[i] : dnan();      // NaN padding: comparisons false
+        for (int k = lane; k <= n; k += 32) lnk[k] = log((double)k);
         __syncwarp();
         double* orow = A.out + (size_t)s * A.ncols;
         int j = 0;
         while (j < A.nd) {
             int left = A.nd - j;
-            if (left >= 6) { entropy_batch<6>(A.descs, j, 6, xd, n, M.sd, orow, lane, lnk, bm); j += 6; }
-            else if (left > 3) { entropy_batch<6>(A.descs, j, left, xd, n, M.sd, orow, lane, lnk, bm); j += left; }
-            else if (left == 3) { entropy_batch<3>(A.descs, j, 3, xd, n, M.sd, orow, lane, lnk, bm); j += 3; }
-            else if (left == 2) { entropy_batch<2>(A.descs, j, 2, xd, n, M.sd, orow, lane, lnk, bm); j += 2; }
-            else { entropy_batch<1>(A.descs, j, 1, xd, n, M.sd, orow, lane, lnk, bm); j += 1; }
+            if (left >= 6) { entropy_batch<6>(A.descs, j, 6, xd, n, M.sd, orow, lane, lnk); j += 6; }
+            else if (left > 3) { entropy_batch<6>(A.descs, j, left, xd, n, M.sd, orow, lane, lnk); j += left; }
+            else if (left == 3) { entropy_batch<3>(A.descs, j, 3, xd, n, M.sd, orow, lane, lnk); j += 3; }
+            else if (left == 2) { entropy_batch<2>(A.descs, j, 2, xd, n, M.sd, orow, lane, lnk); j += 2; }
+            else { entropy_batch<1>(A.descs, j, 1, xd, n, M.sd, orow, lane, lnk); j += 1; }
         }
         __syncwarp();
     }
 }
 
-
 // ---------------------------------------------------------------------------------------------------
-// Rank-space formulation (default for series whose prefix table fits in shared memory).
+// Rank-space formulation (series whose prefix table fits in shared memory).
 // Sort the series once (rank a <-> time index pi(a)).  For a tolerance tau the set { j : |x_i - x_j| <= tau } is a
 // CONTIGUOUS rank interval [lo, hi] around rank(i) (float64 subtraction of float32-origin values is monotone), so
 // the bit row of the bit-tile formulation needs no pair tests at all:
 //     R_i = T[hi + 1] & ~T[lo],      T[k] = { j : rank(j) < k }   (prefix bit vectors in TIME order, built once)
 // and the template counts stay popc(R_i & R_{i+1} >> 1 [& R_{i+2} >> 2]).  The interval ends come from two binary
 // searches per (row, tolerance) with exactly the predicate numpy evaluates ( fl64(x_a - x_b) <= tau ), so the counts
-// are bit-identical to the pair-test formulations above.  O(n^2 / 32) word operations + O(n log n) searches per
+// are bit-identical to the pair-test formulation above.  O(n^2 / 32) word operations + O(n log n) searches per
 // tolerance instead of O(n^2) float64 compares.
 // G warps work on one series (G = 1: warp per series; G > 1: the CTA is one series and shares the table).
 template <int G>
@@ -232,10 +176,14 @@ __device__ __forceinline__ float key_f32(unsigned k) {
 struct RankLayout {            // byte offsets inside one series' working region
     int t_off, s_off, pi_off, rk_off, lh_off, cnt_off, red_off, bytes;
     int lh_stride;             // words between the two interval tables
-    int rs;                    // row stride of T in 32-bit words (multiple of 4; padded to an odd multiple of 16 bytes when pad != 0)
+    int rs;                    // row stride of T in 32-bit words (multiple of 4; an odd multiple of 16 bytes when G > 1)
 };
-__host__ __device__ inline RankLayout rank_layout(int nmax, int G, int pad) {
+// Rows are padded when several warps share one series: an unpadded 128-byte row stride puts every row on the same
+// banks.  With one warp per series they are not: measured on B200 at 1 M x 256, 39.1 ms unpadded (16 warps/SM) vs
+// 39.2 ms padded (12 warps/SM).
+__host__ __device__ inline RankLayout rank_layout(int nmax, int G) {
     RankLayout L;
+    const bool pad = G > 1;
     int n2 = 32;
     while (n2 < nmax) n2 <<= 1;
     const int W = (nmax + 31) >> 5;
@@ -266,7 +214,7 @@ __global__ void __launch_bounds__(G * SPC * 32, (G == 1 ? 4 : (G == 4 ? 4 : 1)))
     const int grp = threadIdx.x / NTHR;                 // series slot inside the CTA
     const int tid = threadIdx.x - grp * NTHR;           // thread inside the series group
     const int gw = tid >> 5;                            // warp inside the series group
-    const RankLayout L = rank_layout(A.npad, G, G > 1 ? 1 : A.rank_pad);
+    const RankLayout L = rank_layout(A.npad, G);
     double* lnk = reinterpret_cast<double*>(smem_raw);                              // log(k), k = 0..npad (CTA-wide)
     unsigned char* base = smem_raw + (((A.npad + 1) * 8 + 15) & ~15) + (size_t)grp * L.bytes;
     unsigned* T = reinterpret_cast<unsigned*>(base + L.t_off);
@@ -564,19 +512,12 @@ __global__ void __launch_bounds__(G * SPC * 32, (G == 1 ? 4 : (G == 4 ? 4 : 1)))
     }
 }
 
-// TSFX_ENTROPY = pairs | tiles | rank (default): which formulation counts the template matches
-static int entropy_mode() {
-    static int mode = -1;
-    if (mode < 0) { const char* e = getenv("TSFX_ENTROPY"); mode = !e ? 2 : (e[0] == 'p' ? 0 : (e[0] == 't' ? 1 : 2)); }
-    return mode;
-}
-
 template <int G, int SPC>
 static cudaError_t launch_rank(const EntropyArgs& A, size_t smem, int ctas_per_sm, cudaStream_t st, int sm_count) {
     cudaError_t e = cudaFuncSetAttribute(k_entropy_rank<G, SPC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int64_t ctas = (A.R.n_series + SPC - 1) / SPC;
-    const int64_t cap = (int64_t)sm_count * ctas_per_sm * grid_waves(16);
+    const int64_t cap = (int64_t)sm_count * ctas_per_sm * 16;
     if (ctas > cap) ctas = cap;
     if (ctas < 1) ctas = 1;
     k_entropy_rank<G, SPC><<<(int)ctas, G * SPC * 32, smem, st>>>(A);
@@ -587,20 +528,13 @@ cudaError_t launch_entropy(const EntropyArgs& A0, int max_len, cudaStream_t st, 
     EntropyArgs A = A0;
     A.npad = (max_len + 3) & ~3;
     A.xpad = ((A.npad + 2 + 31) / 32) * 32 + 32;          // NaN padding up to a whole 32-sample tile / 32-row block
-    const int mode = entropy_mode();
-    A.bittile = mode != 0;
-    if (mode == 2 && max_len < 65000) {
+    if (max_len < 65000) {
         // rank-space kernel: warp per series while four working regions fit three CTAs per SM, then 4 / 16 warps per
         // series with the CTA sharing one prefix table; beyond that (n > ~1100) the pair-test tiles below take over
         const size_t lnk = (((size_t)A.npad + 1) * 8 + 15) & ~(size_t)15;
-        // TSFX_ENTROPY_PAD=1 pads the table rows to an odd multiple of 16 bytes (fewer bank conflicts, fewer resident warps)
-        static int pad = -1;
-        if (pad < 0) { const char* e = getenv("TSFX_ENTROPY_PAD"); pad = (e && e[0] == '1') ? 1 : 0; }
-        A.rank_pad = pad;
-        const size_t s1 = lnk + 4 * (size_t)rank_layout(A.npad, 1, pad).bytes;
-        // several warps per series: rows are always padded (an unpadded 128-byte row stride puts every row on the same banks)
-        const size_t s4 = lnk + (size_t)rank_layout(A.npad, 4, 1).bytes;
-        const size_t s16 = lnk + (size_t)rank_layout(A.npad, 16, 1).bytes;
+        const size_t s1 = lnk + 4 * (size_t)rank_layout(A.npad, 1).bytes;
+        const size_t s4 = lnk + (size_t)rank_layout(A.npad, 4).bytes;
+        const size_t s16 = lnk + (size_t)rank_layout(A.npad, 16).bytes;
         const size_t sm_bytes = 227 * 1024;
         if (s1 <= 75 * 1024) return launch_rank<1, 4>(A, s1, (int)std::min<size_t>(4, sm_bytes / (s1 + 1024)), st, sm_count);
         if (s4 <= 55 * 1024) return launch_rank<4, 1>(A, s4, 4, st, sm_count);

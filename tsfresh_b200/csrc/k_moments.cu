@@ -310,13 +310,13 @@ cudaError_t launch_moments(const MomentsArgs& A, cudaStream_t st, int sm_count) 
     constexpr int SUB = 8, WPC = 8;
     const int64_t per_cta = (int64_t)WPC * (32 / SUB);
     int64_t ctas = (A.R.n_series + per_cta - 1) / per_cta;
-    const int64_t cap = (int64_t)sm_count * 8 * grid_waves(8);
+    const int64_t cap = (int64_t)sm_count * 8 * 8;
     if (ctas > cap) ctas = cap;
     if (ctas < 1) ctas = 1;
     const bool dense = A.R.begin == nullptr && (A.R.dense_len & 3) == 0 && A.R.dense_len >= 4 && A.R.dense_len <= 8 * SUB * 4 &&
                        ((uintptr_t)A.R.values & 15u) == 0;
     if (dense) {
-        const int64_t cap2 = (int64_t)sm_count * 2 * grid_waves(1);          // persistent: two CTAs per SM, prefetching
+        const int64_t cap2 = (int64_t)sm_count * 2;          // persistent: two CTAs per SM, prefetching
         int64_t c2 = (A.R.n_series + per_cta - 1) / per_cta;
         if (c2 > cap2) c2 = cap2;
         k_moments_dense<SUB, WPC, 8><<<(int)c2, WPC * 32, 0, st>>>(A);

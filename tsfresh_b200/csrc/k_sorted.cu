@@ -416,21 +416,8 @@ cudaError_t launch_sorted(const SortedArgs& A0, int max_len, cudaStream_t st, in
     Geometry G;
     if (!plan_geometry(per, 100 * 1024, 8, A.R.n_series, sm_count, A.gscratch, A.gscratch_bytes, &G)) return cudaErrorInvalidConfiguration;
     A.gscratch = G.gscratch;
-    {
-        // TSFX_SORTED_WPC=12: two CTAs of 12 warps per SM instead of three of 8 (same idea as k_basic: the lock-step walk
-        // shares the instruction stream inside a CTA)
-        static int wide = -1;
-        if (wide < 0) { const char* e = getenv("TSFX_SORTED_WPC"); wide = e ? atoi(e) : 0; }
-        if (wide == 12 && !G.gscratch && G.wpc == 8 && per * 12 <= 113 * 1024) {
-            const size_t smem = per * 12;
-            const int64_t ctas = (A.R.n_series + 11) / 12;
-            const int64_t cap = (int64_t)sm_count * grid_waves(4096);
-            cudaError_t e = cudaFuncSetAttribute(k_sorted<12, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            k_sorted<12, false><<<(int)std::max<int64_t>(1, std::min(ctas, cap)), 12 * 32, smem, st>>>(A);
-            return cudaGetLastError();
-        }
-    }
+    // 8-warp CTAs: the 12-warp CTAs that help k_basic measured 23.7 -> 23.8 ms here on B200 at 1 M x 256 (no
+    // instruction-cache pressure in this kernel; profiles/r2_notes.md)
     TSFX_DISPATCH(k_sorted, G, st, A)
     return cudaGetLastError();
 }

@@ -26,30 +26,6 @@ using namespace tsfx;
 
 static std::string g_create_error;
 
-namespace tsfx {
-int grid_waves(int dflt) {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TSFX_GRID_WAVES"); v = e ? atoi(e) : 0; }
-    return v > 0 ? v : dflt;
-}
-int global_above() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TSFX_GLOBAL_ABOVE"); v = e ? atoi(e) : 0; if (v > 227 * 1024 || v < 0) v = 0; }
-    return v;
-}
-int global_ctas_env() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TSFX_GLOBAL_CTAS"); v = e ? atoi(e) : 0; if (v < 1 || v > 16) v = 0; }
-    return v;
-}
-}  // namespace tsfx
-
-static int env_streams() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TSFX_STREAMS"); v = e ? atoi(e) : 1; if (v < 1) v = 1; if (v > 4) v = 4; }
-    return v;
-}
-
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
@@ -178,9 +154,7 @@ struct Stager {
             e = cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming);
             if (e != cudaSuccess) return e;
         }
-        int n = (int)std::thread::hardware_concurrency();
-        const char* env = getenv("TSFX_COPY_THREADS");
-        n = env ? atoi(env) : std::min(8, std::max(1, n / 2));
+        const int n = std::min(8, std::max(1, (int)std::thread::hardware_concurrency() / 2));
         if (n > 1) start(n);
         return cudaSuccess;
     }
@@ -258,8 +232,6 @@ struct tsfx_ctx {
     cudaStream_t s_peer = nullptr;
     cudaEvent_t ev_peer = nullptr;
     cudaStream_t s_in = nullptr, s_out = nullptr;   // copy streams of the pipelined host path
-    cudaStream_t s_side[3] = {nullptr, nullptr, nullptr};   // optional side streams so kernel groups can overlap
-    cudaEvent_t ev_fork = nullptr, ev_join[3] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
 };
 
@@ -369,10 +341,8 @@ extern "C" int tsfx_ctx_create(int device, void* cuda_stream, tsfx_ctx** out) {
     for (int g = 0; g < G_EVENTS; ++g) { CKC(cudaEventCreate(&ctx->ev[g][0])); CKC(cudaEventCreate(&ctx->ev[g][1])); }
     CKC(cudaStreamCreateWithFlags(&ctx->s_in, cudaStreamNonBlocking));
     CKC(cudaStreamCreateWithFlags(&ctx->s_out, cudaStreamNonBlocking));
-    CKC(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
     CKC(cudaStreamCreateWithFlags(&ctx->s_peer, cudaStreamNonBlocking));
     CKC(cudaEventCreateWithFlags(&ctx->ev_peer, cudaEventDisableTiming));
-    for (int i = 0; i < 3; ++i) { CKC(cudaStreamCreateWithFlags(&ctx->s_side[i], cudaStreamNonBlocking)); CKC(cudaEventCreateWithFlags(&ctx->ev_join[i], cudaEventDisableTiming)); }
     for (int i = 0; i < 2; ++i) { CKC(cudaEventCreateWithFlags(&ctx->ev_in[i], cudaEventDisableTiming)); CKC(cudaEventCreateWithFlags(&ctx->ev_done[i], cudaEventDisableTiming)); }
     // decimal threshold table d * 10^k (correctly rounded literals via strtod)
     {
@@ -408,8 +378,6 @@ extern "C" void tsfx_ctx_destroy(tsfx_ctx* ctx) {
     if (ctx->d_dec) cudaFree(ctx->d_dec);
     if (ctx->d_tw) cudaFree(ctx->d_tw);
     for (int g = 0; g < G_EVENTS; ++g) { if (ctx->ev[g][0]) cudaEventDestroy(ctx->ev[g][0]); if (ctx->ev[g][1]) cudaEventDestroy(ctx->ev[g][1]); }
-    for (int i = 0; i < 3; ++i) { if (ctx->s_side[i]) cudaStreamDestroy(ctx->s_side[i]); if (ctx->ev_join[i]) cudaEventDestroy(ctx->ev_join[i]); }
-    if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
     if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
     if (ctx->s_out) cudaStreamDestroy(ctx->s_out);
     for (int i = 0; i < 2; ++i) { if (ctx->ev_in[i]) cudaEventDestroy(ctx->ev_in[i]); if (ctx->ev_done[i]) cudaEventDestroy(ctx->ev_done[i]); }
@@ -531,7 +499,6 @@ extern "C" int tsfx_plan_create(tsfx_ctx* ctx, const tsfx_feature_desc* descs, i
         if (!moments_only_calc(d.calc)) P->basic_moments_only = false;
         if (d.calc == TSFX_SKEWNESS || d.calc == TSFX_KURTOSIS) P->moments_need_high = 1;
     }
-    { const char* e = getenv("TSFX_NO_MOMENTS_KERNEL"); if (e && e[0] == '1') P->basic_moments_only = false; }
     for (int g = 0; g < G_COUNT; ++g) P->n_groups_used += P->host[g].empty() ? 0 : 1;
     if (!final_col.empty()) {
         cudaError_t e = cudaMalloc(&P->d_final_col, final_col.size() * sizeof(int32_t));
@@ -608,7 +575,7 @@ extern "C" int tsfx_set_row_times(tsfx_ctx* ctx, const int64_t* row_time_ns, int
     return TSFX_OK;
 }
 
-static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int max_len, double* d_out, uint32_t flags, int ld = 0) {
+static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int max_len, double* d_final, uint32_t flags, int ld = 0) {
     if (ld <= 0) ld = P->ncols;          // row stride of the caller's matrix
     const bool timing = (flags & TSFX_FLAG_TIMING) != 0;
     for (int g = 0; g < G_EVENTS; ++g) ctx->ev_used[g] = false;
@@ -618,9 +585,10 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
     if (staged == 0) return TSFX_OK;
     CK(ctx->stage.reserve((size_t)R.n_series * staged * sizeof(double)));
     CK(ctx->misc.reserve(max_len > 1024 ? ((size_t)1 << 30) : ((size_t)256 << 20)));      // global working regions for series too long for shared memory
-    double* const d_final = d_out;
-    (void)d_final;
-    if (!P->host[G_SPECTRAL].empty()) {      // FFT twiddle table (filled once, on the main stream, before any fork)
+    // the groups run back to back on ctx->stream, so each may use the whole working region
+    unsigned char* const gscratch = (unsigned char*)ctx->misc.p;
+    const size_t gscratch_bytes = ctx->misc.cap;
+    if (!P->host[G_SPECTRAL].empty()) {      // FFT twiddle table (filled once)
         int p2 = 1;
         while (p2 < max_len) p2 <<= 1;
         if (p2 > max_len) p2 >>= 1;            // largest power of two <= max_len
@@ -628,13 +596,6 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
         int rc = ensure_twiddle(ctx, p2);
         if (rc) return rc;
     }
-    // kernel groups are independent (own staging matrix): optionally spread them over side streams
-    const int nstreams = timing ? 1 : env_streams();
-    if (nstreams > 1) {
-        CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
-        for (int i = 0; i < nstreams - 1; ++i) CK(cudaStreamWaitEvent(ctx->s_side[i], ctx->ev_fork, 0));
-    }
-    int launched = 0;
     bool direct = false;          // the only group wrote the final matrix itself
     ctx->used_moments = false;
     if (max_len < 1) return fail(ctx, TSFX_E_INVALID, "series of length < 1");
@@ -646,14 +607,8 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
         if (P->host[g].empty()) continue;
         if (timing) { CK(cudaEventRecord(ctx->ev[g][0], ctx->stream)); }
         cudaError_t e = cudaSuccess;
-        double* d_out = (double*)ctx->stage.p + (size_t)R.n_series * P->cum[g];      // this group's staging matrix
-        const int sidx = launched++ % nstreams;
-        cudaStream_t gs = (sidx == 0) ? ctx->stream : ctx->s_side[sidx - 1];
+        double* d_stage = (double*)ctx->stage.p + (size_t)R.n_series * P->cum[g];      // this group's staging matrix
         const int g_ncols = (int)P->host[g].size();
-        // global working region: the whole buffer when the groups run back to back, a private slice per group when
-        // they overlap on side streams (concurrent groups must not share working sets)
-        const size_t slice = (nstreams > 1) ? (ctx->misc.cap / G_COUNT) & ~(size_t)255 : ctx->misc.cap;
-        unsigned char* const gs_base = (unsigned char*)ctx->misc.p + (nstreams > 1 ? (size_t)g * slice : 0);
         switch (g) {
             case G_BASIC: {
                 if (P->basic_moments_only) {
@@ -662,15 +617,15 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
                     MomentsArgs M;
                     M.R = R; M.descs = P->dev[g]; M.nd = g_ncols; M.need_high = P->moments_need_high;
                     direct = (P->n_groups_used == 1) && ctx->peer_out.empty() && (P->ncols == g_ncols);
-                    M.out = direct ? d_final : d_out;
+                    M.out = direct ? d_final : d_stage;
                     M.ncols = direct ? ld : g_ncols;
                     M.colmap = direct ? P->d_final_col + P->cum[g] : nullptr;
-                    e = launch_moments(M, gs, ctx->sm_count);
+                    e = launch_moments(M, ctx->stream, ctx->sm_count);
                     ctx->used_moments = true;
                     break;
                 }
                 BasicArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.lag_needed = P->lag_needed;
                 A.nfin = P->basic_nfin;
                 int pac = P->pacf_want >= 0 ? 4 * (P->pacf_want + 1) : 0;
@@ -687,12 +642,12 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
                         }
                 }
                 A.dec = ctx->d_dec;
-                e = launch_basic(A, max_len, gs, ctx->sm_count);
+                e = launch_basic(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_SORTED: {
                 SortedArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.nscr = even(4 * (P->friedrich_r + 2) + 16);
                 A.nfin = P->sorted_nfin;
                 A.ncq = 0;
@@ -701,46 +656,46 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
                     for (const Desc& q : P->host[g])
                         if (q.calc == TSFX_CHANGE_QUANTILES && !(q.p0 == pl && q.p1 == ph)) { ++A.ncq; pl = q.p0; ph = q.p1; }
                 }
-                e = launch_sorted(A, max_len, gs, ctx->sm_count);
+                e = launch_sorted(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_SPECTRAL: {
                 SpectralArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.twiddle = ctx->d_tw; A.tw_n = ctx->tw_n;
                 A.tables = P->d_tables; A.table_off = P->d_toff; A.table_half = P->d_thalf;
                 A.need_fft = P->need_fft; A.need_welch = P->need_welch;
                 A.max_hist = P->fourier_bins;
                 A.nfft = P->spectral_nfft;
-                e = launch_spectral(A, max_len, gs, ctx->sm_count);
+                e = launch_spectral(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_LA: {
                 LaArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.nscr = P->max_ar_k;
-                e = launch_la(A, max_len, gs, ctx->sm_count);
+                e = launch_la(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_ENTROPY: {
                 EntropyArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
-                e = launch_entropy(A, max_len, gs, ctx->sm_count);
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
+                e = launch_entropy(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_SEQ: {
                 SeqArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.nscr = (P->max_lz_bins > 0 ? 1 : 0) | (P->max_perm_dim > 0 ? 2 : 0) | (P->max_cwt_peaks_n << 8) |
                          (std::min(P->n_lz, 255) << 16) | (std::min(P->max_lz_bins, 255) << 24);
-                e = launch_seq(A, max_len, gs, ctx->sm_count);
+                e = launch_seq(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
             case G_PEAKS: {
                 SeqArgs A;
-                A.R = R; A.gscratch = gs_base; A.gscratch_bytes = slice; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_out; A.ncols = g_ncols;
+                A.R = R; A.gscratch = gscratch; A.gscratch_bytes = gscratch_bytes; A.descs = P->dev[g]; A.nd = (int)P->host[g].size(); A.out = d_stage; A.ncols = g_ncols;
                 A.nscr = (P->max_cwt_peaks_n << 8);
-                e = launch_peaks(A, max_len, gs, ctx->sm_count);
+                e = launch_peaks(A, max_len, ctx->stream, ctx->sm_count);
                 break;
             }
         }
@@ -749,11 +704,6 @@ static int run_groups(tsfx_ctx* ctx, const tsfx_plan* P, const SeriesRef& R, int
         ctx->launches += 1;
         if (timing) { CK(cudaEventRecord(ctx->ev[g][1], ctx->stream)); ctx->ev_used[g] = true; }
     }
-    if (nstreams > 1)
-        for (int i = 0; i < nstreams - 1; ++i) {
-            CK(cudaEventRecord(ctx->ev_join[i], ctx->s_side[i]));
-            CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[i], 0));
-        }
     if (!direct) {   // scatter the staging matrices into the caller's [n_series x ncols] matrix
         if (timing) { CK(cudaEventRecord(ctx->ev[G_COUNT][0], ctx->stream)); }
         AssembleArgs A;

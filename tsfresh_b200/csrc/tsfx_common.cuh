@@ -135,11 +135,4 @@ __device__ __forceinline__ Moments moments(const float* xs, int n, double* xc, i
     return M;
 }
 
-// ---------------------------------------------------------------- launch geometry helper (host)
-struct WarpLaunch {
-    int warps_per_cta;
-    size_t smem_bytes;
-    int grid;
-};
-
 }  // namespace tsfx

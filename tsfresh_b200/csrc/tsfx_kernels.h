@@ -8,12 +8,6 @@
 
 namespace tsfx {
 
-// CTAs per SM in a launch (each CTA loops over its share of the series).  TSFX_GRID_WAVES overrides the
-// per-kernel default (tuning knob, read once).
-int grid_waves(int dflt);
-int global_above();
-int global_ctas_env();
-
 struct Geometry { int wpc; size_t smem; int grid; unsigned char* gscratch; };
 
 // Chooses warps per CTA / grid for a warp-per-series kernel needing `per` bytes per warp.  Shared memory when it
@@ -24,15 +18,13 @@ inline bool plan_geometry(size_t per, size_t budget, int maxw, int64_t n_series,
     // Working sets above `prefer_global_above` bytes per warp run from the global (L2-resident) region even though
     // they would fit in shared memory: measured on B200, the latency-bound PEAKS / SEQ kernels are up to 5x faster
     // that way at 1024 samples because shared memory would limit them to 2-4 warps per SM (profiles/r1_notes.md).
-    // TSFX_GLOBAL_ABOVE=<bytes> overrides the per-kernel threshold for experiments.
-    const size_t thr = global_above() > 0 ? (size_t)global_above() : prefer_global_above;
-    if (per <= thr && per <= 227 * 1024) {
+    if (per <= prefer_global_above && per <= 227 * 1024) {
         size_t w = budget / per;
         int wpc = w >= 8 ? 8 : w >= 4 ? 4 : w >= 2 ? 2 : 1;
         while (wpc > maxw) wpc >>= 1;
         G->wpc = wpc;
         G->smem = per * wpc;
-        int64_t cap = (int64_t)sm_count * grid_waves(4096);
+        int64_t cap = (int64_t)sm_count * 4096;      // CTAs per SM: each CTA loops over its share of the series
         int64_t ctas = (n_series + wpc - 1) / wpc;
         G->grid = (int)(ctas < cap ? (ctas < 1 ? 1 : ctas) : cap);
         G->gscratch = nullptr;
@@ -43,8 +35,8 @@ inline bool plan_geometry(size_t per, size_t budget, int maxw, int64_t n_series,
     if (max_ctas < 1) { wpc = 1; max_ctas = gs ? gs_bytes / per : 0; }
     if (max_ctas < 1) return false;
     int64_t ctas = (n_series + wpc - 1) / wpc;
-    // CTAs per SM in global-region mode: TSFX_GLOBAL_CTAS, else the kernel's own choice, else 4
-    int64_t cap = (int64_t)sm_count * (global_ctas_env() > 0 ? global_ctas_env() : global_ctas > 0 ? global_ctas : 4);
+    // CTAs per SM in global-region mode: the kernel's own choice, else 4
+    int64_t cap = (int64_t)sm_count * (global_ctas > 0 ? global_ctas : 4);
     if ((int64_t)max_ctas < cap) cap = (int64_t)max_ctas;
     G->wpc = wpc;
     G->smem = 0;
@@ -177,8 +169,7 @@ struct LaArgs {
 cudaError_t launch_la(const LaArgs& A, int max_len, cudaStream_t st, int sm_count);
 
 struct EntropyArgs {
-    int rank_pad;              // rank-space kernel: pad the prefix-table rows (bank conflicts vs. occupancy)
-    int xpad, bittile;         // padded sample count; 1 = bit-tile counting (default), 0 = pair sweep (TSFX_ENTROPY=pairs)
+    int xpad;                  // padded sample count of the bit-tile kernel
     SeriesRef R;
     unsigned char* gscratch;     // global scratch (API) -> set to nullptr by the launcher when shared memory is used
     size_t gscratch_bytes;
